@@ -15,7 +15,9 @@ also carries the figures BASELINE.json names beside it: G1 MSM at 2^20 points (M
 a 2^20 Groth16 proof, GM17, a 64-node PCD tree, and -- N > 1 -- one MSM and one proof sharded over the GPUs through the
 library's own NCCL exchange.  Every timed figure is first checked against the CPU oracle (outside the timed regions).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR`: after the timed steps, the four proofs of the last one go to DIR/<proof>.npy (see dump_outputs).
 
 `--impl reference`: the CPU arm.  The reference (Rust, un-vendored arkworks crates) cannot be built here, so this times
 oracle/c (the C++ restatement of the same algorithms in the shape arkworks runs them: 5x64 CIOS, arkworks' Pippenger
@@ -255,10 +257,9 @@ class PcdStep:
         return [draw_rs(rng, part["inst"]["p"]) for part in self.parts]
 
     def step_dev(self, rs):
-        out = None
-        for part, (r, s) in zip(self.parts, rs):
-            out = part["g"].create_proof_dev(part["idx"], part["z_dev"].data_ptr(), r, s)
-        return out
+        """the step's four proofs, in proving order"""
+        return [part["g"].create_proof_dev(part["idx"], part["z_dev"].data_ptr(), r, s)
+                for part, (r, s) in zip(self.parts, rs)]
 
     def step_host(self, rs):
         c = self.ctx
@@ -335,12 +336,14 @@ def run_gpu(args, rank, local_rank, world):
     barrier()
     e0.record(stream)
     for i in range(args.steps):
-        step.step_dev(rs[args.warmup + i])
+        proofs = step.step_dev(rs[args.warmup + i])
     e1.record(stream)
     barrier()
     ms_dev = max_over_ranks(e0.elapsed_time(e1))
     ctx._check(ctx.lib.pcdgpu_profile_read(ctx.h, ms, units, spans, ctypes.byref(launches)))
     n_launches = int(launches.value)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step.parts, proofs)
 
     # ---- timed region 2: end to end through the C ABI with host buffers ---------------------------------------
     step.step_host(rs[0])  # untimed: grows the host path's staging scratch
@@ -505,6 +508,17 @@ def run_gpu(args, rank, local_rank, world):
     emit(line)
 
 
+def dump_outputs(out_dir, parts, proofs):
+    """The proofs of the last timed step as out_dir/<proof label>.npy: the affine limbs (A, then B, then C; Montgomery
+    coordinates, as create_proof_dev returns them), one row per u64 limb holding its low and high 32-bit halves as
+    float64, which represents them exactly.  The inputs are seeded, so two builds can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    for part, proof in zip(parts, proofs):
+        limbs = proof.affine_limbs().astype(np.uint64)
+        halves = np.stack([limbs & np.uint64(0xFFFFFFFF), limbs >> np.uint64(32)], axis=1).astype(np.float64)
+        np.save(os.path.join(out_dir, part["label"] + ".npy"), halves)
+
+
 def tree_figure(args, ctx, step, stream, rank, world, barrier, max_over_ranks, log):
     """BASELINE config 5: a binary tree of PCD nodes, every node one full step (its four proofs), children before
     parents, nodes of a round spread round-robin over the GPUs, each node drawing from its own generator
@@ -516,7 +530,7 @@ def tree_figure(args, ctx, step, stream, rank, world, barrier, max_over_ranks, l
 
     def prove_node(node, child_proofs, rng):
         rs = [(tree.draw_scalar(rng, part["inst"]["p"]), tree.draw_scalar(rng, part["inst"]["p"])) for part in step.parts]
-        return step.step_dev(rs).affine_limbs().tobytes()
+        return step.step_dev(rs)[-1].affine_limbs().tobytes()
 
     tree.prove_tree(min(n, 3), prove_node, rank, world)  # warm-up (and the collective's first call)
     barrier()
@@ -896,7 +910,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernel-figures", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the MSM / NTT size sweeps")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the four proofs of the last timed step to DIR/<proof>.npy (rank 0; GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's proofs")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
