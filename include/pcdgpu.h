@@ -323,6 +323,39 @@ int pcdgpu_msm_bases_sharded_dev(pcdgpu_ctx* ctx, const pcdgpu_bases* slice, con
  * larger root", 6 = infinity on the last byte): 152 B (MNT4) / 190 B (MNT6).  out: >= 190 bytes. */
 int pcdgpu_serialize_proof(pcdgpu_ctx* ctx, int pairing, const void* proof_affine, uint8_t* out, size_t* out_len);
 
+/* ---- pairings and proof verification (ark-ec PairingEngine::pairing, ark-groth16 / ark-gm17 verifier.rs) -------
+ * Reduced ate pairings of MNT4-298 (GT = Fq4 = Fq2[v]/(v^2 - u), 160 B) and MNT6-298 (GT = Fq6 = Fq3[v]/(v^2 - u),
+ * 240 B); GT bytes are arkworks' in-memory QuadExtField {c0, c1}, Montgomery limbs.  One GPU thread per pair / proof:
+ * a single call takes milliseconds, throughput comes from large batches.  These calls take the same
+ * one-caller-at-a-time guard as the provers.
+ * Input rules of the verifiers: a proof with a coordinate >= p or a point off its curve gets out_ok = 0 (not an
+ * error).  Membership of B in the prime-order subgroup of G2 is NOT checked -- arkworks' verify does not check it
+ * either, its deserialization does: callers that take proofs from untrusted bytes check it there. */
+/* out_gt[i] = e(g1[i], g2[i]); a point at infinity (x = y = 0) gives 1 */
+int pcdgpu_pairing(pcdgpu_ctx* ctx, int pairing, const void* g1, const void* g2, size_t n, void* out_gt);
+/* ark-groth16 prepare_verifying_key of VerifyingKey {alpha_g1, beta_g2, gamma_g2, delta_g2, gamma_abc_g1[num_inputs]}
+ * (num_inputs counts the constant: gamma_abc_g1.len()).  Runs on the GPU: line coefficients of -gamma and -delta and
+ * e(alpha, beta).  A key point off its curve or with a coordinate >= p: PCDGPU_E_ARG. */
+typedef struct pcdgpu_groth16_pvk pcdgpu_groth16_pvk;
+int pcdgpu_groth16_pvk_create(pcdgpu_ctx* ctx, int pairing, const void* alpha_g1, const void* beta_g2,
+                              const void* gamma_g2, const void* delta_g2, const void* gamma_abc_g1, size_t num_inputs,
+                              pcdgpu_groth16_pvk** out);
+void pcdgpu_groth16_pvk_free(pcdgpu_groth16_pvk* pvk);
+/* verify_with_processed_vk for n proofs: proofs = n x (A || B || C) in pcdgpu_groth16_prove's layout, inputs =
+ * n x (num_inputs - 1) Montgomery Fr elements (ark's &[E::Fr]; may be NULL when num_inputs = 1); out_ok[i] = 1 / 0.
+ * n = 0 returns PCDGPU_OK. */
+int pcdgpu_groth16_verify_batch(pcdgpu_ctx* ctx, const pcdgpu_groth16_pvk* pvk, const void* proofs, const void* inputs,
+                                size_t n, uint8_t* out_ok);
+/* the same for GM17: VerifyingKey {h_g2, g_alpha_g1, h_beta_g2, g_gamma_g1, h_gamma_g2, query[num_inputs]}; both of
+ * ark-gm17's pairing equations are checked per proof */
+typedef struct pcdgpu_gm17_pvk pcdgpu_gm17_pvk;
+int pcdgpu_gm17_pvk_create(pcdgpu_ctx* ctx, int pairing, const void* h_g2, const void* g_alpha_g1,
+                           const void* h_beta_g2, const void* g_gamma_g1, const void* h_gamma_g2, const void* query,
+                           size_t num_inputs, pcdgpu_gm17_pvk** out);
+void pcdgpu_gm17_pvk_free(pcdgpu_gm17_pvk* pvk);
+int pcdgpu_gm17_verify_batch(pcdgpu_ctx* ctx, const pcdgpu_gm17_pvk* pvk, const void* proofs, const void* inputs,
+                             size_t n, uint8_t* out_ok);
+
 /* ---- profiling ----------------------------------------------------------------------------------
  * CUDA-event spans around the library's kernel groups, on the context's stream.  Classes (array
  * index): 0 MSM digit/sort, 1 the accumulate kernel of a large G1 MSM, 2 same G2 over Fq2, 3 MSM bucket reduction,

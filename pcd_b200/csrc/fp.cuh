@@ -33,6 +33,11 @@ PCD_HD u32 fp_mod_opaque(int i) {  // i = FP_LIMBS: -p^-1 mod 2^32
   return i < FP_LIMBS ? P::mod(i) : P::INV;
 }
 
+#if defined(PCDGPU_HOSTEMU)
+// base-field products executed by this host thread: the work model of the pairing code (tests/hostemu)
+inline thread_local unsigned long long pcd_emu_products = 0;
+#endif
+
 template <class P>
 struct Fp {
   u32 l[FP_LIMBS];
@@ -175,6 +180,9 @@ struct Fp {
   }
 
   PCD_HD friend Fp operator*(const Fp& a, const Fp& b) {
+#if defined(PCDGPU_HOSTEMU)
+    ++pcd_emu_products;
+#endif
     return mul_cc(a, b);
   }
   // carry-chain product (IMAD.WIDE.U32.X rows)

@@ -47,7 +47,11 @@ EXPORTS = [
     "pcdgpu_vec_powers_dev", "pcdgpu_vec_gather_dev", "pcdgpu_poly_eval_dev", "pcdgpu_poly_divide_vanishing_dev",
     "pcdgpu_poly_divide_linear_dev", "pcdgpu_ntt_general_dev", "pcdgpu_csr_upload", "pcdgpu_csr_free",
     "pcdgpu_csr_matvec_dev", "pcdgpu_kzg_commit_dev",
+    "pcdgpu_pairing", "pcdgpu_groth16_pvk_create", "pcdgpu_groth16_pvk_free", "pcdgpu_groth16_verify_batch",
+    "pcdgpu_gm17_pvk_create", "pcdgpu_gm17_pvk_free", "pcdgpu_gm17_verify_batch",
 ]
+#: u64 limbs of a GT element per pairing (arkworks' QuadExtField over Fq2 / Fq3)
+GT_LIMBS = {MNT4_298: 20, MNT6_298: 30}
 COMM_ID_BYTES = 128
 
 
@@ -167,6 +171,15 @@ def load():
     lib.pcdgpu_csr_free.restype = None
     lib.pcdgpu_csr_matvec_dev.argtypes = [vp, vp, vp, vp]
     lib.pcdgpu_kzg_commit_dev.argtypes = [vp, vp, sz, vp, sz, vp, vp, sz, vp]
+    lib.pcdgpu_pairing.argtypes = [vp, ci, vp, vp, sz, vp]
+    lib.pcdgpu_groth16_pvk_create.argtypes = [vp, ci] + [vp] * 5 + [sz, ctypes.POINTER(vp)]
+    lib.pcdgpu_groth16_pvk_free.argtypes = [vp]
+    lib.pcdgpu_groth16_pvk_free.restype = None
+    lib.pcdgpu_groth16_verify_batch.argtypes = [vp, vp, vp, vp, sz, vp]
+    lib.pcdgpu_gm17_pvk_create.argtypes = [vp, ci] + [vp] * 6 + [sz, ctypes.POINTER(vp)]
+    lib.pcdgpu_gm17_pvk_free.argtypes = [vp]
+    lib.pcdgpu_gm17_pvk_free.restype = None
+    lib.pcdgpu_gm17_verify_batch.argtypes = [vp, vp, vp, vp, sz, vp]
     _lib = lib
     return lib
 
@@ -260,6 +273,17 @@ class Context:
 
     def ntt_dev(self, field: int, d_ptr: int, log_n: int, inverse: bool = False, coset: bool = False):
         self._check(self.lib.pcdgpu_ntt_dev(self.h, field, ctypes.c_void_p(d_ptr), log_n, int(inverse), int(coset)))
+
+    # ---- pairings ----
+    def pairing(self, pairing: int, g1: np.ndarray, g2: np.ndarray) -> np.ndarray:
+        """e(g1[i], g2[i]) for every row: (n, GT_LIMBS[pairing]) u64 limbs (ark-ec PairingEngine::pairing)"""
+        g1 = _u64(g1, AFFINE_LIMBS[G1_OF[pairing]])
+        g2 = _u64(g2, AFFINE_LIMBS[G2_OF[pairing]])
+        if g1.shape[0] != g2.shape[0]:
+            raise ValueError("g1 and g2 hold different numbers of points")
+        out = np.zeros((g1.shape[0], GT_LIMBS[pairing]), dtype=np.uint64)
+        self._check(self.lib.pcdgpu_pairing(self.h, pairing, _p(g1), _p(g2), g1.shape[0], _p(out)))
+        return out
 
     # ---- MSM ----
     def msm(self, curve: int, bases: np.ndarray, scalars: np.ndarray) -> np.ndarray:

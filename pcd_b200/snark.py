@@ -149,9 +149,125 @@ class ProverIndex:
             pass
 
 
-class Groth16:
-    """`Groth16<E>` as the reference binds it (SNARK + CircuitSpecificSetupSNARK); only `prove` and
-    its building blocks run on the GPU.  Setup / verify stay with the CPU implementation on the
+# ---- verification (ark-groth16 / ark-gm17 verifier.rs) ------------------------------------------------------------
+@dataclass
+class VerifyingKey:
+    """ark-groth16 `VerifyingKey<E>`; gamma_abc_g1 has one point per public input plus the constant's."""
+
+    pairing: int
+    alpha_g1: np.ndarray
+    beta_g2: np.ndarray
+    gamma_g2: np.ndarray
+    delta_g2: np.ndarray
+    gamma_abc_g1: np.ndarray
+
+
+@dataclass
+class GM17VerifyingKey:
+    """ark-gm17 `VerifyingKey<E>`; query has one point per public input plus the constant's."""
+
+    pairing: int
+    h_g2: np.ndarray
+    g_alpha_g1: np.ndarray
+    h_beta_g2: np.ndarray
+    g_gamma_g1: np.ndarray
+    h_gamma_g2: np.ndarray
+    query: np.ndarray
+
+
+class PreparedVerifyingKey:
+    """A verifying key processed on the GPU (pcdgpu_groth16_pvk / pcdgpu_gm17_pvk): the line coefficients of its G2
+    points and e(alpha, beta) stay in device memory."""
+
+    def __init__(self, ctx: L.Context, pairing: int, gm17: bool, handle, num_inputs: int):
+        self.ctx, self.pairing, self.gm17, self.h, self.num_inputs = ctx, pairing, gm17, handle, num_inputs
+
+    def close(self):
+        if getattr(self, "h", None):
+            free = self.ctx.lib.pcdgpu_gm17_pvk_free if self.gm17 else self.ctx.lib.pcdgpu_groth16_pvk_free
+            free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _points(a, curve) -> np.ndarray:
+    return np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, L.AFFINE_LIMBS[curve])
+
+
+def _verify_batch(ctx: L.Context, pvk: PreparedVerifyingKey, gm17: bool, xs, proofs) -> np.ndarray:
+    if pvk.gm17 != gm17:
+        raise ValueError("the prepared key belongs to the other proof system")
+    width = L.AFFINE_LIMBS[L.G1_OF[pvk.pairing]] * 2 + L.AFFINE_LIMBS[L.G2_OF[pvk.pairing]]
+    if isinstance(proofs, np.ndarray):
+        pr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(-1, width)
+    else:
+        pr = np.ascontiguousarray([p.affine_limbs() for p in proofs], dtype=np.uint64).reshape(-1, width)
+    n = pr.shape[0]
+    ni = pvk.num_inputs - 1
+    x = np.ascontiguousarray(xs, dtype=np.uint64).reshape(n, -1) if n else np.zeros((0, 5), dtype=np.uint64)
+    if n and x.shape[1] != 5 * ni:
+        # ark: SynthesisError::MalformedVerifyingKey for a public-input count the key does not have
+        raise L.PcdGpuError(-1, "the key takes %d public inputs, got %d" % (ni, x.shape[1] // 5))
+    ok = np.zeros(n, dtype=np.uint8)
+    if n == 0:
+        return ok.astype(bool)
+    lib = ctx.lib
+    fn = lib.pcdgpu_gm17_verify_batch if gm17 else lib.pcdgpu_groth16_verify_batch
+    ctx._check(fn(ctx.h, pvk.h, L._p(pr), L._p(x) if ni else None, n, L._p(ok)))
+    return ok.astype(bool)
+
+
+def _process_vk(ctx: L.Context, pairing: int, gm17: bool, vk) -> PreparedVerifyingKey:
+    """ark-groth16 / ark-gm17 prepare_verifying_key, on the GPU (a key point off its curve: PcdGpuError -1)"""
+    g1, g2 = L.G1_OF[pairing], L.G2_OF[pairing]
+    if gm17:
+        pts = [_points(vk.h_g2, g2), _points(vk.g_alpha_g1, g1), _points(vk.h_beta_g2, g2),
+               _points(vk.g_gamma_g1, g1), _points(vk.h_gamma_g2, g2), _points(vk.query, g1)]
+        create = ctx.lib.pcdgpu_gm17_pvk_create
+    else:
+        pts = [_points(vk.alpha_g1, g1), _points(vk.beta_g2, g2), _points(vk.gamma_g2, g2), _points(vk.delta_g2, g2),
+               _points(vk.gamma_abc_g1, g1)]
+        create = ctx.lib.pcdgpu_groth16_pvk_create
+    if vk.pairing != pairing:
+        raise ValueError("verifying key of another pairing")
+    h = ctypes.c_void_p()
+    ctx._check(create(ctx.h, pairing, *[L._p(a) for a in pts], pts[-1].shape[0], ctypes.byref(h)))
+    return PreparedVerifyingKey(ctx, pairing, gm17, h, pts[-1].shape[0])
+
+
+class _Verifier:
+    """verify / verify_with_processed_vk / verify_batch shared by Groth16 and GM17 (GM17 sets _GM17)"""
+
+    _GM17 = False
+
+    def process_vk(self, vk) -> PreparedVerifyingKey:
+        return _process_vk(self.ctx, self.pairing, self._GM17, vk)
+
+    def verify_batch(self, pvk: PreparedVerifyingKey, xs, proofs) -> np.ndarray:
+        """one verdict per proof: xs = n x (num_inputs - 1) Montgomery Fr elements, proofs = Proof objects or an
+        (n, A || B || C) limb array"""
+        return _verify_batch(self.ctx, pvk, self._GM17, xs, proofs)
+
+    def verify_with_processed_vk(self, pvk: PreparedVerifyingKey, x, proof: Proof) -> bool:
+        x = np.ascontiguousarray(x, dtype=np.uint64).reshape(1, -1)
+        return bool(_verify_batch(self.ctx, pvk, self._GM17, x, [proof])[0])
+
+    def verify(self, vk, x, proof: Proof) -> bool:
+        pvk = self.process_vk(vk)
+        try:
+            return self.verify_with_processed_vk(pvk, x, proof)
+        finally:
+            pvk.close()
+
+
+class Groth16(_Verifier):
+    """`Groth16<E>` as the reference binds it (SNARK + CircuitSpecificSetupSNARK): `prove` and its building
+    blocks, `process_vk` and verification run on the GPU.  Setup stays with the CPU implementation on the
     Rust side of the boundary (SURVEY.md 3.3, 3.4)."""
 
     def __init__(self, ctx: L.Context, pairing: int):
@@ -298,9 +414,12 @@ class GM17ProverIndex:
             pass
 
 
-class GM17:
+class GM17(_Verifier):
     """`GM17<E>` as the reference binds it (/root/reference/tests/mnt4_gm17.rs:27-28): `prove` and its building
-    blocks on the GPU; setup / verify stay with the CPU implementation on the Rust side of the boundary."""
+    blocks, `process_vk` and verification on the GPU; setup stays with the CPU implementation on the Rust side of
+    the boundary."""
+
+    _GM17 = True
 
     def __init__(self, ctx: L.Context, pairing: int):
         self.ctx, self.pairing = ctx, pairing
@@ -354,3 +473,4 @@ class GM17:
     def serialize(self, proof: Proof) -> bytes:
         """ark-serialize canonical (compressed) bytes of `Proof {a, b, c}`: 152 B (MNT4-298) / 190 B (MNT6-298)."""
         return self.ctx.serialize_proof(self.pairing, proof.affine_limbs())
+

@@ -12,6 +12,8 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] pub struct pcdgpu_pk { _p: [u8; 0] }
 #[repr(C)] pub struct pcdgpu_gm17_pk { _p: [u8; 0] }
 #[repr(C)] pub struct pcdgpu_csr { _p: [u8; 0] }
+#[repr(C)] pub struct pcdgpu_groth16_pvk { _p: [u8; 0] }
+#[repr(C)] pub struct pcdgpu_gm17_pvk { _p: [u8; 0] }
 
 pub const PCDGPU_OK: c_int = 0;
 pub const PCDGPU_E_ARG: c_int = -1;
@@ -110,6 +112,13 @@ extern "C" {
     pub fn pcdgpu_msm_bases_sharded(ctx: *mut pcdgpu_ctx, slice: *const pcdgpu_bases, scalars: *const c_void, n: usize, out_affine: *mut c_void) -> c_int;
     pub fn pcdgpu_msm_bases_sharded_dev(ctx: *mut pcdgpu_ctx, slice: *const pcdgpu_bases, d_scalars: *const c_void, scalars_mont: c_int, n: usize, d_out_affine: *mut c_void) -> c_int;
     pub fn pcdgpu_serialize_proof(ctx: *mut pcdgpu_ctx, pairing: c_int, proof_affine: *const c_void, out: *mut u8, out_len: *mut usize) -> c_int;
+    pub fn pcdgpu_pairing(ctx: *mut pcdgpu_ctx, pairing: c_int, g1: *const c_void, g2: *const c_void, n: usize, out_gt: *mut c_void) -> c_int;
+    pub fn pcdgpu_groth16_pvk_create(ctx: *mut pcdgpu_ctx, pairing: c_int, alpha_g1: *const c_void, beta_g2: *const c_void, gamma_g2: *const c_void, delta_g2: *const c_void, gamma_abc_g1: *const c_void, num_inputs: usize, out: *mut *mut pcdgpu_groth16_pvk) -> c_int;
+    pub fn pcdgpu_groth16_pvk_free(pvk: *mut pcdgpu_groth16_pvk);
+    pub fn pcdgpu_groth16_verify_batch(ctx: *mut pcdgpu_ctx, pvk: *const pcdgpu_groth16_pvk, proofs: *const c_void, inputs: *const c_void, n: usize, out_ok: *mut u8) -> c_int;
+    pub fn pcdgpu_gm17_pvk_create(ctx: *mut pcdgpu_ctx, pairing: c_int, h_g2: *const c_void, g_alpha_g1: *const c_void, h_beta_g2: *const c_void, g_gamma_g1: *const c_void, h_gamma_g2: *const c_void, query: *const c_void, num_inputs: usize, out: *mut *mut pcdgpu_gm17_pvk) -> c_int;
+    pub fn pcdgpu_gm17_pvk_free(pvk: *mut pcdgpu_gm17_pvk);
+    pub fn pcdgpu_gm17_verify_batch(ctx: *mut pcdgpu_ctx, pvk: *const pcdgpu_gm17_pvk, proofs: *const c_void, inputs: *const c_void, n: usize, out_ok: *mut u8) -> c_int;
     pub fn pcdgpu_profile_enable(ctx: *mut pcdgpu_ctx, on: c_int) -> c_int;
     pub fn pcdgpu_profile_read(ctx: *mut pcdgpu_ctx, ms: *mut f64, units: *mut f64, spans: *mut u64, launches: *mut u64) -> c_int;
     pub fn pcdgpu_profile_timeline(ctx: *mut pcdgpu_ctx, t0_ms: *mut f64, t1_ms: *mut f64, cls: *mut c_int, cap: usize, count: *mut usize) -> c_int;

@@ -11,7 +11,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(ROOT, "rust", "pcdgpu-sys", "src", "lib.rs")
 TMAP = {"int": "c_int", "size_t": "usize", "uint32_t": "u32", "uint64_t": "u64", "uint8_t": "u8", "double": "f64",
         "void": "c_void", "char": "c_char"}
-HANDLES = {"pcdgpu_ctx", "pcdgpu_bases", "pcdgpu_r1cs", "pcdgpu_pk", "pcdgpu_gm17_pk", "pcdgpu_csr"}
+HANDLES = {"pcdgpu_ctx", "pcdgpu_bases", "pcdgpu_r1cs", "pcdgpu_pk", "pcdgpu_gm17_pk", "pcdgpu_csr", "pcdgpu_groth16_pvk",
+           "pcdgpu_gm17_pvk"}
 HEAD = '''// UNCOMPILED SOURCE (see ../../README.md).  The `extern "C"` block is GENERATED from include/pcdgpu.h by
 // tools/gen_rust_sys.py: one declaration per exported function, same order, same names.
 // Encodings (include/pcdgpu.h): field element = 5 x u64 little-endian Montgomery limbs (ark-ff Fp320 / BigInteger320);
@@ -26,6 +27,8 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] pub struct pcdgpu_pk { _p: [u8; 0] }
 #[repr(C)] pub struct pcdgpu_gm17_pk { _p: [u8; 0] }
 #[repr(C)] pub struct pcdgpu_csr { _p: [u8; 0] }
+#[repr(C)] pub struct pcdgpu_groth16_pvk { _p: [u8; 0] }
+#[repr(C)] pub struct pcdgpu_gm17_pvk { _p: [u8; 0] }
 
 pub const PCDGPU_OK: c_int = 0;
 pub const PCDGPU_E_ARG: c_int = -1;
