@@ -330,7 +330,8 @@ int pcdgpu_serialize_proof(pcdgpu_ctx* ctx, int pairing, const void* proof_affin
  * one-caller-at-a-time guard as the provers.
  * Input rules of the verifiers: a proof with a coordinate >= p or a point off its curve gets out_ok = 0 (not an
  * error).  Membership of B in the prime-order subgroup of G2 is NOT checked -- arkworks' verify does not check it
- * either, its deserialization does: callers that take proofs from untrusted bytes check it there. */
+ * either, its deserialization does: callers that take proofs from untrusted bytes pass the bytes to
+ * pcdgpu_deserialize_proofs or pcdgpu_*_verify_batch_serialized below, which check it. */
 /* out_gt[i] = e(g1[i], g2[i]); a point at infinity (x = y = 0) gives 1 */
 int pcdgpu_pairing(pcdgpu_ctx* ctx, int pairing, const void* g1, const void* g2, size_t n, void* out_gt);
 /* ark-groth16 prepare_verifying_key of VerifyingKey {alpha_g1, beta_g2, gamma_g2, delta_g2, gamma_abc_g1[num_inputs]}
@@ -355,6 +356,23 @@ int pcdgpu_gm17_pvk_create(pcdgpu_ctx* ctx, int pairing, const void* h_g2, const
 void pcdgpu_gm17_pvk_free(pcdgpu_gm17_pvk* pvk);
 int pcdgpu_gm17_verify_batch(pcdgpu_ctx* ctx, const pcdgpu_gm17_pvk* pvk, const void* proofs, const void* inputs,
                              size_t n, uint8_t* out_ok);
+
+/* ---- proofs from bytes (ark-serialize CanonicalDeserialize for Proof {a, b, c}, checked) -------------------------
+ * bytes = n x pcdgpu_serialize_proof's encoding (152 B MNT4 / 190 B MNT6, rows back to back).  A point is valid when
+ * every coordinate chunk (flag bits masked) is < p, not both flag bits are set, and either the infinity flag is set
+ * (the point is infinity, whatever x is) or x^3 + a x + b has a square root (the one flag bit 7 selects); B must also
+ * satisfy [r]B = O (G2 subgroup membership; both G1 groups have cofactor 1).  One GPU thread per proof.
+ * out_affine = n x (A || B || C) in pcdgpu_groth16_prove's layout, all zero for an invalid proof; out_ok[i] = 1 / 0.
+ * An invalid proof is a verdict, not an error.  n = 0 returns PCDGPU_OK; an unknown pairing or a null pointer with
+ * n > 0: PCDGPU_E_ARG. */
+int pcdgpu_deserialize_proofs(pcdgpu_ctx* ctx, int pairing, const uint8_t* bytes, size_t n, void* out_affine,
+                              uint8_t* out_ok);
+/* deserialize and verify in one call, the proofs staying on the device in between: out_ok[i] = the bytes are a valid
+ * proof && it verifies (pcdgpu_*_verify_batch's rules for inputs and n) */
+int pcdgpu_groth16_verify_batch_serialized(pcdgpu_ctx* ctx, const pcdgpu_groth16_pvk* pvk, const uint8_t* bytes,
+                                           const void* inputs, size_t n, uint8_t* out_ok);
+int pcdgpu_gm17_verify_batch_serialized(pcdgpu_ctx* ctx, const pcdgpu_gm17_pvk* pvk, const uint8_t* bytes,
+                                        const void* inputs, size_t n, uint8_t* out_ok);
 
 /* ---- profiling ----------------------------------------------------------------------------------
  * CUDA-event spans around the library's kernel groups, on the context's stream.  Classes (array

@@ -33,7 +33,7 @@
 namespace pcdgpu {
 
 // ---- Result / Error (ark-relations SynthesisError + backend errors) --------------------------------
-enum class ErrorKind { None, Unsupported, AssignmentMissing, MalformedKey, DomainTooLarge, Backend };
+enum class ErrorKind { None, Unsupported, AssignmentMissing, MalformedKey, DomainTooLarge, Backend, InvalidData };
 struct Error {
   ErrorKind kind = ErrorKind::None;
   int code = 0;          // PCDGPU_E_* for Backend errors
@@ -296,6 +296,33 @@ class Groth16 {
     res.value.resize(len);
     return res;
   }
+
+  // CanonicalDeserialize for Proof<E> (checked, on the GPU): bytes that are not a valid proof give
+  // ErrorKind::InvalidData (ark's SerializationError::InvalidData)
+  static Result<ProofT> deserialize(const std::vector<uint8_t>& bytes) {
+    Result<ProofT> res;
+    if (bytes.size() != E::PROOF_BYTES) {
+      res.error = {ErrorKind::InvalidData, 0, "a compressed proof has the wrong length"};
+      return res;
+    }
+    auto ctx = Backend::get();
+    if (!ctx) { res.error = ctx.error; return res; }
+    std::vector<uint64_t> out(2 * E::G1_LIMBS + E::G2_LIMBS);
+    uint8_t ok = 0;
+    int rc = pcdgpu_deserialize_proofs(ctx.value, E::PAIRING, bytes.data(), 1, out.data(), &ok);
+    if (rc != PCDGPU_OK) {
+      res.error = {ErrorKind::Backend, rc, pcdgpu_last_error(ctx.value)};
+      return res;
+    }
+    if (!ok) {
+      res.error = {ErrorKind::InvalidData, 0, "invalid proof encoding"};
+      return res;
+    }
+    std::memcpy(res.value.a.data(), out.data(), 8 * E::G1_LIMBS);
+    std::memcpy(res.value.b.data(), out.data() + E::G1_LIMBS, 8 * E::G2_LIMBS);
+    std::memcpy(res.value.c.data(), out.data() + E::G1_LIMBS + E::G2_LIMBS, 8 * E::G1_LIMBS);
+    return res;
+  }
 };
 
 // ---- ark-gm17 data structures and GM17<E>: SNARK + CircuitSpecificSetupSNARK -------------------------------
@@ -429,6 +456,7 @@ class GM17 {
   }
 
   static Result<std::vector<uint8_t>> serialize(const ProofT& p) { return Groth16<E>::serialize(p); }
+  static Result<ProofT> deserialize(const std::vector<uint8_t>& bytes) { return Groth16<E>::deserialize(bytes); }
 };
 
 }  // namespace pcdgpu

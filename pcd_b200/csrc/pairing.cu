@@ -11,7 +11,7 @@
 #include <cstring>
 
 #include "common.cuh"
-#include "pairing.cuh"
+#include "deserialize.cuh"
 
 #define PAIR_CHECK_ARG(ctx, cond, msg)      \
   do {                                      \
@@ -58,11 +58,11 @@ __global__ void vk_prepare_kernel(const AffinePoint<typename PP::E>* g2, PrepSpe
 template <class PP>
 __global__ void __launch_bounds__(PAIR_BLOCK) groth16_verify_kernel(Groth16Pvk<PP> vk, const char* __restrict__ proofs,
                                                                     const typename PP::Fr* __restrict__ x, size_t n,
-                                                                    unsigned char* __restrict__ ok) {
+                                                                    unsigned char* __restrict__ ok, bool gated) {
   typedef AffinePoint<typename PP::B> A1;
   typedef AffinePoint<typename PP::E> A2;
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  if (i >= n || (gated && !ok[i])) return;
   const char* p = proofs + i * (2 * sizeof(A1) + sizeof(A2));
   ok[i] = groth16_verify_one<PP>(vk, *reinterpret_cast<const A1*>(p), *reinterpret_cast<const A2*>(p + sizeof(A1)),
                                  *reinterpret_cast<const A1*>(p + sizeof(A1) + sizeof(A2)),
@@ -72,11 +72,11 @@ __global__ void __launch_bounds__(PAIR_BLOCK) groth16_verify_kernel(Groth16Pvk<P
 template <class PP>
 __global__ void __launch_bounds__(PAIR_BLOCK) gm17_verify_kernel(GM17Pvk<PP> vk, const char* __restrict__ proofs,
                                                                  const typename PP::Fr* __restrict__ x, size_t n,
-                                                                 unsigned char* __restrict__ ok) {
+                                                                 unsigned char* __restrict__ ok, bool gated) {
   typedef AffinePoint<typename PP::B> A1;
   typedef AffinePoint<typename PP::E> A2;
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  if (i >= n || (gated && !ok[i])) return;
   const char* p = proofs + i * (2 * sizeof(A1) + sizeof(A2));
   ok[i] = gm17_verify_one<PP>(vk, *reinterpret_cast<const A1*>(p), *reinterpret_cast<const A2*>(p + sizeof(A1)),
                               *reinterpret_cast<const A1*>(p + sizeof(A1) + sizeof(A2)),
@@ -187,9 +187,11 @@ static void vk_free(VkCommon* v) {
   }
 }
 
-// Stages n proofs (and their inputs) and runs the scheme's kernel; out_ok on the host when it returns.
+// Stages n proofs (and their inputs) and runs the scheme's kernel; out_ok on the host when it returns.  serialized:
+// the proofs are compressed bytes, deserialized on the device into the rows the verifier reads; a proof whose bytes
+// are invalid keeps verdict 0 (the verify kernel skips it).
 static int verify_batch(pcdgpu_ctx* ctx, const VkCommon* v, bool gm17, const void* proofs, const void* inputs, size_t n,
-                        uint8_t* out_ok) {
+                        uint8_t* out_ok, bool serialized = false) {
   PAIR_CHECK_ARG(ctx, v && (n == 0 || (proofs && out_ok && (v->num_inputs == 1 || inputs))), "null pointer");
   if (n == 0) return PCDGPU_OK;
   PAIR_CHECK_ARG(ctx, v->device == ctx->device, "the key was processed on another device");
@@ -198,26 +200,38 @@ static int verify_batch(pcdgpu_ctx* ctx, const VkCommon* v, bool gm17, const voi
   PAIR_CHECK_ARG(ctx, guard.ok, "the context is running a call on another host thread (one context per thread)");
   const bool m4 = v->pairing == PCDGPU_MNT4_298;
   const size_t proof_bytes = m4 ? 320 : 400;
+  const size_t ser_bytes = serialized ? n * (m4 ? 152 : 190) : 0;
+  const size_t ok_bytes = (n + 255) & ~(size_t)255;
   const size_t x_bytes = n * (v->num_inputs - 1) * 40;
   void *dp, *dx, *dok;
   PCD_TRY(ctx->scratch(SLOT_IO, n * proof_bytes, &dp));
   PCD_TRY(ctx->scratch(SLOT_IO2, x_bytes + 16, &dx));
-  PCD_TRY(ctx->scratch(SLOT_MISC, n + 16, &dok));
+  PCD_TRY(ctx->scratch(SLOT_MISC, ok_bytes + ser_bytes, &dok));
   cudaStream_t st = ctx->stream;
-  PCD_CUDA(ctx, cudaMemcpyAsync(dp, proofs, n * proof_bytes, cudaMemcpyHostToDevice, st));
+  if (serialized) {
+    unsigned char* dser = (unsigned char*)dok + ok_bytes;
+    PCD_CUDA(ctx, cudaMemcpyAsync(dser, proofs, ser_bytes, cudaMemcpyHostToDevice, st));
+    PCD_TRY(pcd_deserialize_proofs_dev(ctx, v->pairing, dser, n, dp, (unsigned char*)dok));
+  } else {
+    PCD_CUDA(ctx, cudaMemcpyAsync(dp, proofs, n * proof_bytes, cudaMemcpyHostToDevice, st));
+  }
   if (x_bytes) PCD_CUDA(ctx, cudaMemcpyAsync(dx, inputs, x_bytes, cudaMemcpyHostToDevice, st));
   if (m4 && !gm17)
     groth16_verify_kernel<PairMnt4><<<grid_of(n), PAIR_BLOCK, 0, st>>>(groth16_view<PairMnt4>(v), (const char*)dp,
-                                                                      (const FpR4*)dx, n, (unsigned char*)dok);
+                                                                      (const FpR4*)dx, n, (unsigned char*)dok,
+                                                                      serialized);
   else if (!gm17)
     groth16_verify_kernel<PairMnt6><<<grid_of(n), PAIR_BLOCK, 0, st>>>(groth16_view<PairMnt6>(v), (const char*)dp,
-                                                                      (const FpQ4*)dx, n, (unsigned char*)dok);
+                                                                      (const FpQ4*)dx, n, (unsigned char*)dok,
+                                                                      serialized);
   else if (m4)
     gm17_verify_kernel<PairMnt4><<<grid_of(n), PAIR_BLOCK, 0, st>>>(gm17_view<PairMnt4>(v), (const char*)dp,
-                                                                   (const FpR4*)dx, n, (unsigned char*)dok);
+                                                                   (const FpR4*)dx, n, (unsigned char*)dok,
+                                                                   serialized);
   else
     gm17_verify_kernel<PairMnt6><<<grid_of(n), PAIR_BLOCK, 0, st>>>(gm17_view<PairMnt6>(v), (const char*)dp,
-                                                                   (const FpQ4*)dx, n, (unsigned char*)dok);
+                                                                   (const FpQ4*)dx, n, (unsigned char*)dok,
+                                                                   serialized);
   PCD_CUDA(ctx, cudaGetLastError());
   PCD_CUDA(ctx, cudaMemcpyAsync(out_ok, dok, n, cudaMemcpyDeviceToHost, st));
   PCD_CUDA(ctx, cudaStreamSynchronize(st));
@@ -339,6 +353,18 @@ int pcdgpu_gm17_verify_batch(pcdgpu_ctx* ctx, const pcdgpu_gm17_pvk* pvk, const 
                              size_t n, uint8_t* out_ok) {
   if (!ctx) return PCDGPU_E_ARG;
   return verify_batch(ctx, pvk, true, proofs, inputs, n, out_ok);
+}
+
+int pcdgpu_groth16_verify_batch_serialized(pcdgpu_ctx* ctx, const pcdgpu_groth16_pvk* pvk, const uint8_t* bytes,
+                                           const void* inputs, size_t n, uint8_t* out_ok) {
+  if (!ctx) return PCDGPU_E_ARG;
+  return verify_batch(ctx, pvk, false, bytes, inputs, n, out_ok, true);
+}
+
+int pcdgpu_gm17_verify_batch_serialized(pcdgpu_ctx* ctx, const pcdgpu_gm17_pvk* pvk, const uint8_t* bytes,
+                                        const void* inputs, size_t n, uint8_t* out_ok) {
+  if (!ctx) return PCDGPU_E_ARG;
+  return verify_batch(ctx, pvk, true, bytes, inputs, n, out_ok, true);
 }
 
 }  // extern "C"

@@ -271,7 +271,8 @@ PCD_HD GT<PP> pairing(const AffinePoint<typename PP::B>& p, const AffinePoint<ty
   return final_exponentiation<PP>(miller_loop<PP>(a));
 }
 
-// ---- input checks (ark-serialize's: canonical coordinates, on the curve; G2 subgroup membership is NOT checked) ----
+// ---- input checks (ark-serialize's: canonical coordinates, on the curve; G2 subgroup membership is checked by the
+// deserialization of deserialize.cuh, not here) ----
 template <class B>
 PCD_HD bool base_canonical(const B& x) {
   for (int i = FP_LIMBS - 1; i >= 0; i--)
@@ -280,6 +281,15 @@ PCD_HD bool base_canonical(const B& x) {
 }
 template <class F> struct BaseOf { typedef typename F::Base T; };
 template <class P> struct BaseOf<Fp<P>> { typedef Fp<P> T; };
+// x^3 + a x + b on C
+template <class C>
+PCD_HD typename C::F curve_rhs(const typename C::F& x) {
+  typedef typename C::F F;
+  F b;
+  u32* bw = reinterpret_cast<u32*>(&b);
+  for (int i = 0; i < F::WORDS; i++) bw[i] = C::Gen::coeff_b(i);
+  return (x.sqr() + C::mul_a(F::one())) * x + b;
+}
 template <class C>
 PCD_HD bool valid_point(const AffinePoint<typename C::F>& p) {
   typedef typename C::F F;
@@ -288,10 +298,7 @@ PCD_HD bool valid_point(const AffinePoint<typename C::F>& p) {
   for (int i = 0; i < 2 * F::WORDS / FP_LIMBS; i++)
     if (!base_canonical(c[i])) return false;
   if (p.is_inf()) return true;
-  F b;
-  u32* bw = reinterpret_cast<u32*>(&b);
-  for (int i = 0; i < F::WORDS; i++) bw[i] = C::Gen::coeff_b(i);
-  return p.y.sqr() == (p.x.sqr() + C::mul_a(F::one())) * p.x + b;
+  return p.y.sqr() == curve_rhs<C>(p.x);
 }
 
 // gamma_abc[0] + sum_i x_i gamma_abc[i + 1] (x: Montgomery scalar-field elements), affine

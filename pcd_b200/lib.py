@@ -49,9 +49,12 @@ EXPORTS = [
     "pcdgpu_csr_matvec_dev", "pcdgpu_kzg_commit_dev",
     "pcdgpu_pairing", "pcdgpu_groth16_pvk_create", "pcdgpu_groth16_pvk_free", "pcdgpu_groth16_verify_batch",
     "pcdgpu_gm17_pvk_create", "pcdgpu_gm17_pvk_free", "pcdgpu_gm17_verify_batch",
+    "pcdgpu_deserialize_proofs", "pcdgpu_groth16_verify_batch_serialized", "pcdgpu_gm17_verify_batch_serialized",
 ]
 #: u64 limbs of a GT element per pairing (arkworks' QuadExtField over Fq2 / Fq3)
 GT_LIMBS = {MNT4_298: 20, MNT6_298: 30}
+#: bytes of a compressed proof (pcdgpu_serialize_proof) per pairing
+PROOF_BYTES = {MNT4_298: 152, MNT6_298: 190}
 COMM_ID_BYTES = 128
 
 
@@ -180,6 +183,9 @@ def load():
     lib.pcdgpu_gm17_pvk_free.argtypes = [vp]
     lib.pcdgpu_gm17_pvk_free.restype = None
     lib.pcdgpu_gm17_verify_batch.argtypes = [vp, vp, vp, vp, sz, vp]
+    lib.pcdgpu_deserialize_proofs.argtypes = [vp, ci, vp, sz, vp, vp]
+    lib.pcdgpu_groth16_verify_batch_serialized.argtypes = [vp, vp, vp, vp, sz, vp]
+    lib.pcdgpu_gm17_verify_batch_serialized.argtypes = [vp, vp, vp, vp, sz, vp]
     _lib = lib
     return lib
 
@@ -360,6 +366,15 @@ class Context:
         n = ctypes.c_size_t()
         self._check(self.lib.pcdgpu_serialize_proof(self.h, pairing, _p(proof_affine), _p(out), ctypes.byref(n)))
         return out[:n.value].tobytes()
+
+    def deserialize_proofs(self, pairing: int, rows: np.ndarray):
+        """checked ark-serialize deserialization of n compressed proofs ((n, PROOF_BYTES[pairing]) uint8) ->
+        ((n, A || B || C) affine limbs, zero rows for invalid proofs; (n,) bool verdicts)"""
+        width = 2 * AFFINE_LIMBS[G1_OF[pairing]] + AFFINE_LIMBS[G2_OF[pairing]]
+        out = np.zeros((rows.shape[0], width), dtype=np.uint64)
+        ok = np.zeros(rows.shape[0], dtype=np.uint8)
+        self._check(self.lib.pcdgpu_deserialize_proofs(self.h, pairing, _p(rows), rows.shape[0], _p(out), _p(ok)))
+        return out, ok.astype(bool)
 
 
 class Bases:

@@ -199,11 +199,13 @@ def _points(a, curve) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, L.AFFINE_LIMBS[curve])
 
 
-def _verify_batch(ctx: L.Context, pvk: PreparedVerifyingKey, gm17: bool, xs, proofs) -> np.ndarray:
+def _verify_batch(ctx: L.Context, pvk: PreparedVerifyingKey, gm17: bool, xs, proofs, serialized=False) -> np.ndarray:
     if pvk.gm17 != gm17:
         raise ValueError("the prepared key belongs to the other proof system")
     width = L.AFFINE_LIMBS[L.G1_OF[pvk.pairing]] * 2 + L.AFFINE_LIMBS[L.G2_OF[pvk.pairing]]
-    if isinstance(proofs, np.ndarray):
+    if serialized:
+        pr = _proof_rows(pvk.pairing, proofs)
+    elif isinstance(proofs, np.ndarray):
         pr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(-1, width)
     else:
         pr = np.ascontiguousarray([p.affine_limbs() for p in proofs], dtype=np.uint64).reshape(-1, width)
@@ -217,9 +219,28 @@ def _verify_batch(ctx: L.Context, pvk: PreparedVerifyingKey, gm17: bool, xs, pro
     if n == 0:
         return ok.astype(bool)
     lib = ctx.lib
-    fn = lib.pcdgpu_gm17_verify_batch if gm17 else lib.pcdgpu_groth16_verify_batch
+    if serialized:
+        fn = lib.pcdgpu_gm17_verify_batch_serialized if gm17 else lib.pcdgpu_groth16_verify_batch_serialized
+    else:
+        fn = lib.pcdgpu_gm17_verify_batch if gm17 else lib.pcdgpu_groth16_verify_batch
     ctx._check(fn(ctx.h, pvk.h, L._p(pr), L._p(x) if ni else None, n, L._p(ok)))
     return ok.astype(bool)
+
+
+def _proof_rows(pairing: int, data) -> np.ndarray:
+    """compressed proofs as one (n, PROOF_BYTES[pairing]) uint8 array: a 2-D array, or a sequence of bytes objects"""
+    width = L.PROOF_BYTES[pairing]
+    if isinstance(data, np.ndarray):
+        rows = np.ascontiguousarray(data, dtype=np.uint8)
+        if rows.ndim != 2 or rows.shape[1] != width:
+            raise ValueError("compressed proofs over this pairing are rows of %d bytes, got shape %s" % (
+                width, rows.shape))
+        return rows
+    data = [bytes(b) for b in data]
+    for b in data:
+        if len(b) != width:
+            raise ValueError("a compressed proof over this pairing is %d bytes, got %d" % (width, len(b)))
+    return np.frombuffer(b"".join(data), dtype=np.uint8).reshape(-1, width).copy()
 
 
 def _process_vk(ctx: L.Context, pairing: int, gm17: bool, vk) -> PreparedVerifyingKey:
@@ -263,6 +284,28 @@ class _Verifier:
             return self.verify_with_processed_vk(pvk, x, proof)
         finally:
             pvk.close()
+
+    def deserialize_batch(self, data):
+        """ark-serialize CanonicalDeserialize (checked) of n compressed proofs, on the GPU: data = an (n, 152 / 190)
+        uint8 array or a sequence of bytes.  Returns ((n, A || B || C) affine limbs, zero rows for invalid proofs;
+        (n,) bool mask of valid proofs)."""
+        rows = _proof_rows(self.pairing, data)
+        return self.ctx.deserialize_proofs(self.pairing, rows)
+
+    def deserialize(self, data: bytes) -> Proof:
+        """one compressed proof -> Proof; ValueError when the bytes are not a valid proof (ark's
+        SerializationError::InvalidData): a coordinate >= p, both flags, no square root, B outside the subgroup"""
+        limbs, ok = self.deserialize_batch([data])
+        if not ok[0]:
+            raise ValueError("invalid proof encoding")
+        g1, g2 = L.AFFINE_LIMBS[L.G1_OF[self.pairing]], L.AFFINE_LIMBS[L.G2_OF[self.pairing]]
+        row = limbs[0]
+        return Proof(self.pairing, row[:g1].copy(), row[g1:g1 + g2].copy(), row[g1 + g2:].copy())
+
+    def verify_batch_serialized(self, pvk: PreparedVerifyingKey, xs, data) -> np.ndarray:
+        """verify_batch for compressed proofs (deserialize_batch's input): one verdict per proof, true when the bytes
+        deserialize to a valid proof and it verifies; the proofs stay on the GPU in between"""
+        return _verify_batch(self.ctx, pvk, self._GM17, xs, data, serialized=True)
 
 
 class Groth16(_Verifier):

@@ -119,6 +119,9 @@ extern "C" {
     pub fn pcdgpu_gm17_pvk_create(ctx: *mut pcdgpu_ctx, pairing: c_int, h_g2: *const c_void, g_alpha_g1: *const c_void, h_beta_g2: *const c_void, g_gamma_g1: *const c_void, h_gamma_g2: *const c_void, query: *const c_void, num_inputs: usize, out: *mut *mut pcdgpu_gm17_pvk) -> c_int;
     pub fn pcdgpu_gm17_pvk_free(pvk: *mut pcdgpu_gm17_pvk);
     pub fn pcdgpu_gm17_verify_batch(ctx: *mut pcdgpu_ctx, pvk: *const pcdgpu_gm17_pvk, proofs: *const c_void, inputs: *const c_void, n: usize, out_ok: *mut u8) -> c_int;
+    pub fn pcdgpu_deserialize_proofs(ctx: *mut pcdgpu_ctx, pairing: c_int, bytes: *const u8, n: usize, out_affine: *mut c_void, out_ok: *mut u8) -> c_int;
+    pub fn pcdgpu_groth16_verify_batch_serialized(ctx: *mut pcdgpu_ctx, pvk: *const pcdgpu_groth16_pvk, bytes: *const u8, inputs: *const c_void, n: usize, out_ok: *mut u8) -> c_int;
+    pub fn pcdgpu_gm17_verify_batch_serialized(ctx: *mut pcdgpu_ctx, pvk: *const pcdgpu_gm17_pvk, bytes: *const u8, inputs: *const c_void, n: usize, out_ok: *mut u8) -> c_int;
     pub fn pcdgpu_profile_enable(ctx: *mut pcdgpu_ctx, on: c_int) -> c_int;
     pub fn pcdgpu_profile_read(ctx: *mut pcdgpu_ctx, ms: *mut f64, units: *mut f64, spans: *mut u64, launches: *mut u64) -> c_int;
     pub fn pcdgpu_profile_timeline(ctx: *mut pcdgpu_ctx, t0_ms: *mut f64, t1_ms: *mut f64, cls: *mut c_int, cap: usize, count: *mut usize) -> c_int;

@@ -4,7 +4,11 @@
 inputs (2 public inputs); the host clock runs around the synchronous call, after one warm-up call of the same size,
 and every timed call's verdicts must all be true.
 
-    python tools/bench_verify.py [--batches 1,64,1024,16384] [--reps 3] [--out bench_verify.json]
+--serialized adds, next to each verify_batch row (op "verify"), the same proofs as compressed bytes (152 / 190 B,
+serialized by the oracle): deserialize_batch alone (op "deserialize", once per pairing) and verify_batch_serialized
+(op "verify_serialized").
+
+    python tools/bench_verify.py [--batches 1,64,1024,16384] [--reps 3] [--serialized] [--out bench_verify.json]
 """
 import argparse
 import json
@@ -19,6 +23,7 @@ for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
 
 import numpy as np  # noqa: E402
 
+import deserialize_helpers as dh  # noqa: E402
 import pcd_b200  # noqa: E402
 import synth  # noqa: E402
 import verify_helpers as vh  # noqa: E402
@@ -38,6 +43,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batches", default="1,64,1024,16384")
     ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--serialized", action="store_true")
     ap.add_argument("--out", default="")
     a = ap.parse_args()
     batches = [int(b) for b in a.batches.split(",")]
@@ -51,22 +57,32 @@ def main():
             vk = pcd_b200.GM17VerifyingKey(**vh.gm17_vk(inst)) if gm17 else pcd_b200.VerifyingKey(**vh.groth16_vk(inst))
             pvk = v.process_vk(vk)
             base_p, base_x = vh.simulated(inst, min(nmax, 2048), 77 + pid, gm17)
+            base_b = np.stack([np.frombuffer(dh.proof_bytes(pid, r), dtype=np.uint8) for r in base_p]) \
+                if a.serialized else None
+            ops = [("verify", lambda p, b, x: v.verify_batch(pvk, x, p))]
+            if a.serialized:
+                if not gm17:
+                    ops.append(("deserialize", lambda p, b, x: v.deserialize_batch(b)[1]))
+                ops.append(("verify_serialized", lambda p, b, x: v.verify_batch_serialized(pvk, x, b)))
             for n in batches:
                 reps = -(-n // base_p.shape[0])
                 proofs = np.ascontiguousarray(np.concatenate([base_p] * reps)[:n])
                 xs = np.ascontiguousarray(np.concatenate([base_x] * reps)[:n])
-                assert v.verify_batch(pvk, xs, proofs).all()  # warm-up, same shape
-                ts = []
-                for _ in range(a.reps):
-                    t0 = time.perf_counter()
-                    ok = v.verify_batch(pvk, xs, proofs)
-                    ts.append(time.perf_counter() - t0)
-                    assert ok.all(), "a valid proof was rejected"
-                t = min(ts)
-                res["results"].append(dict(pairing="mnt4_298" if pid == 0 else "mnt6_298",
-                                           scheme="gm17" if gm17 else "groth16", batch=n, ms_per_call=t * 1e3,
-                                           ms_per_call_all=[x * 1e3 for x in ts], proofs_per_s=n / t))
-                print(json.dumps(res["results"][-1]), file=sys.stderr, flush=True)
+                blobs = np.ascontiguousarray(np.concatenate([base_b] * reps)[:n]) if a.serialized else None
+                for op, fn in ops:
+                    assert fn(proofs, blobs, xs).all()  # warm-up, same shape
+                    ts = []
+                    for _ in range(a.reps):
+                        t0 = time.perf_counter()
+                        ok = fn(proofs, blobs, xs)
+                        ts.append(time.perf_counter() - t0)
+                        assert ok.all(), "a valid proof was rejected"
+                    t = min(ts)
+                    res["results"].append(dict(pairing="mnt4_298" if pid == 0 else "mnt6_298",
+                                               scheme="gm17" if gm17 else "groth16", op=op, batch=n,
+                                               ms_per_call=t * 1e3, ms_per_call_all=[x * 1e3 for x in ts],
+                                               proofs_per_s=n / t))
+                    print(json.dumps(res["results"][-1]), file=sys.stderr, flush=True)
             pvk.close()
     ctx.close()
     line = json.dumps(res)
