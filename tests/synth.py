@@ -71,13 +71,15 @@ def mont_limbs(vals, fp):
     return np.frombuffer(b"".join(o.fp_to_mont_bytes(v, fp) for v in vals), dtype="<u8").copy().reshape(-1, 5)
 
 
-def make_instance(pairing_id, m, seed=20261017, bitlike=0.3, num_inputs=2):
+def make_instance(pairing_id, m, seed=20261017, bitlike=0.3, num_inputs=2, r1cs_z=None):
     """Satisfiable R1CS + assignment + Groth16 key with known trapdoor.  Returns a dict with the CSR
     matrices, z (Montgomery limbs), the key as numpy arrays (PK_FIELDS), and the python-side objects
-    needed for the trapdoor check."""
+    needed for the trapdoor check.  r1cs_z = (R1CS, assignment) replaces the synthetic system (m, bitlike
+    and num_inputs are then ignored)."""
     pairing = PAIRINGS[pairing_id]
     fp = pairing.fr
-    r1cs, z = o.synthetic_r1cs(fp, m, num_inputs=num_inputs, seed=seed, bitlike=bitlike)
+    r1cs, z = r1cs_z or o.synthetic_r1cs(fp, m, num_inputs=num_inputs, seed=seed, bitlike=bitlike)
+    m = r1cs.num_constraints
     t = o.groth16_setup_scalars(pairing, r1cs, seed=seed + 100)
     g1, g2 = codec.G1_OF[pairing_id], codec.G2_OF[pairing_id]
     G1, G2 = generator_limbs(g1), generator_limbs(g2)
@@ -122,12 +124,14 @@ def trapdoor_proof(inst, r, s):
     return np.concatenate([A, B, Cc])
 
 
-def make_gm17_instance(pairing_id, m, seed=20261017, bitlike=0.3, num_inputs=2):
-    """Satisfiable R1CS + assignment + GM17 key with known trapdoor (c_oracle.GM17_PK_FIELDS as numpy arrays)."""
+def make_gm17_instance(pairing_id, m, seed=20261017, bitlike=0.3, num_inputs=2, r1cs_z=None):
+    """Satisfiable R1CS + assignment + GM17 key with known trapdoor (c_oracle.GM17_PK_FIELDS as numpy arrays);
+    r1cs_z as in make_instance."""
     pairing = PAIRINGS[pairing_id]
     fp = pairing.fr
     p = fp.p
-    r1cs, z = o.synthetic_r1cs(fp, m, num_inputs=num_inputs, seed=seed, bitlike=bitlike)
+    r1cs, z = r1cs_z or o.synthetic_r1cs(fp, m, num_inputs=num_inputs, seed=seed, bitlike=bitlike)
+    m = r1cs.num_constraints
     t = o.gm17_setup_scalars(pairing, r1cs, seed=seed + 100)
     g1, g2 = codec.G1_OF[pairing_id], codec.G2_OF[pairing_id]
     G1, G2 = generator_limbs(g1), generator_limbs(g2)
